@@ -5,6 +5,7 @@ Contract (one JSON line on stdout from rank 0):
     python bench.py --gpus N --steps K --warmup W                    # sm_100a kernels behind the drop-in modules
     python bench.py --impl reference --gpus N --steps K --warmup W   # the oracle restatement on the host cores (CPU arm)
     python bench.py --impl reference-gpu ...                         # the same reference-style op chain, eager torch on the B200
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's loss / gradients / parameters as DIR/*.npy
 
 Workloads (``--workload``; BASELINE.json ``configs``):
     qm9      [1] (default, the config the metric is quoted on) 128 molecules x ~18 atoms, radius 5 A, Lmax=2,
@@ -147,6 +148,20 @@ def measured_peaks():
             d = json.load(f)
         return float(d["hbm_gbs"]), float(d["bf16_tflops"]) / 2.0, "measured (MEASURED_PEAKS.json: hbm_gbs, bf16_tflops / 2)"
     return 6650.0, 1125.0, "fallback (B200_PROFILING.md: 6.65 TB/s, 2.25 PFLOP/s bf16 / 2)"
+
+
+def dump_outputs(out_dir: str, arrays, max_elems: int = 1 << 22):
+    """Write each array as ``<out_dir>/<name>.npy``, flattened.  An array of more than ``max_elems`` elements is replaced
+    by a fixed, seeded sample of that many of its elements, so two builds' dumps compare position for position and the
+    three arrays of a step stay well under 64 MB."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.reshape(-1)
+        if t.numel() > max_elems:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:max_elems].sort().values
+            t = t[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy())
 
 
 def ncu_traffic(kernel: str):
@@ -497,12 +512,16 @@ def run_ours(args):
     if mark:
         torch.cuda.cudart().cudaProfilerStart()
     if use_graph:
-        ms_step, _ = timed(args.steps, from_host=False, profile=None)
+        ms_step, last_step_loss = timed(args.steps, from_host=False, profile=None)
     else:
-        ms_step, _ = timed(args.steps, from_host=False, profile=None, fn=step_eager)
+        ms_step, last_step_loss = timed(args.steps, from_host=False, profile=None, fn=step_eager)
     if mark:
         torch.cuda.cudart().cudaProfilerStop()
     clocks = sampler.stop() if sampler else None
+    # what the last timed step handed back (the loss) and left behind (its averaged gradients, the parameters after its
+    # AdamW update), copied before the e2e pass below trains on; float32, as the step computes them
+    last_step = ({"loss": last_step_loss.detach().float().cpu(), "grad": bucket.flat.float().cpu(),
+                  "params": opt.flat.float().cpu()} if args.dump_outputs else None)
     ms_e2e, last_loss = timed(args.steps if args.stream <= 1 else max(args.steps, len(hosts)), from_host=True, profile=None,
                               stream=args.stream > 1)
 
@@ -595,6 +614,8 @@ def run_ours(args):
             "loss": last_loss, "grad_bucket_bytes": bucket.nbytes,
         }
         print(json.dumps(line), flush=True)
+        if last_step is not None:
+            dump_outputs(args.dump_outputs, last_step)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -613,9 +634,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--graph", dest="graph", action="store_true", default=True)
     ap.add_argument("--no-graph", dest="graph", action="store_false")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last one's loss, gradients and updated parameters as DIR/<name>.npy")
     args = ap.parse_args()
     if args.stream > 1 and args.workload != "qm9":
         ap.error("--stream is implemented for the qm9 workload")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs is implemented for --impl ours")
     if args.impl in ("reference", "reference-gpu"):
         run_reference(args)
     else:
